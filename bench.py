@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the PCM -> spectrum -> pixels hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 Default workload (BASELINE.json configs[1], `--config headline`): module `bars`, setbufsize 4096 ("4096-pt FFT"),
 1920x1080 RGBA8, 1024 independent synthetic 22050 Hz stereo streams PER GPU (weak scaling: the batch is sharded
@@ -135,6 +135,30 @@ def config_block(wl, batch, world, p=None, fb_slots=None):
             "batch_per_gpu": batch, "streams_total": batch * world, "parallelism": f"stream-sharded x{world}, no collective"}
 
 
+DUMP_STREAMS = 16          # streams whose outputs --dump-outputs writes
+DUMP_PIXELS = 1 << 17      # pixels per dumped frame (the same seeded positions in every stream)
+
+
+def dump_outputs(out_dir, r, batch):
+    """What the last timed update handed its caller, for output-by-output comparison of two builds: the frames of a seeded
+    sample of streams at a seeded sample of pixel positions.  With a framebuffer ring (fb_slots < batch) only the last
+    `slots` streams still hold their frame, so the sample is drawn from those.  The timed path runs with lazy_smooth = 1,
+    where glava_b200_spectrum() / _textures() hold only the bins the module samples and the rest is stale (glava_b200.h):
+    those are not outputs of this path, and two builds may differ there without any pixel differing, so they are not
+    written.  float32 / float64 only, about 34 MB at the headline configuration."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    p = r.params
+    slots = p.fb_slots if 0 < p.fb_slots < batch else batch
+    rng = np.random.default_rng(0)
+    streams = np.sort(rng.choice(np.arange(batch - slots, batch), size=min(DUMP_STREAMS, slots), replace=False))
+    pixels = np.sort(rng.choice(p.h * p.w, size=min(DUMP_PIXELS, p.h * p.w), replace=False))
+    frames = np.stack([r.readback(int(s)).reshape(-1, 4)[pixels] for s in streams]).astype(np.float32)
+    out = {"stream_index": streams.astype(np.float64), "frame_pixel_index": pixels.astype(np.float64), "frames_rgba8": frames}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args, wl, rank, world):
     """reference arm: the reference's own rd_update (CPU FFT + its GL passes and module shaders on Mesa llvmpipe) on all host
     cores, one GLava renderer per core; a step = every core renders FPW frames of the same workload"""
@@ -177,7 +201,11 @@ def main():
     ap.add_argument("--batch", type=int, default=env_int("GLAVA_BENCH_BATCH", 0), help="streams per GPU (0: the workload's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the lazy_smooth=0 and full-ring legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what their last step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     wl = workload(args.config)
 
@@ -275,6 +303,8 @@ def main():
     t_sampler = time.perf_counter()
     time.sleep(0.25)
     ms_dev, kt, launches = device_leg(r, K)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r, batch)
     # the raster kernel alone (no spectrum kernel co-running): modified=0 re-rasters the last spectrum
     r.set_timing(True)
     for _ in range(10):

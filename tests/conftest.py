@@ -32,12 +32,37 @@ def orc_pm(built):
     return Oracle("pm")
 
 
+def pytest_sessionfinish(session, exitstatus):
+    from tests import reference_record
+    reference_record.save()
+
+
 @pytest.fixture(scope="session")
-def ref(built):
+def ref_live(built):
+    """the reference's compiled transforms themselves, for tests that run them on the reference's own shader tree (their
+    results are its source text and are not stored)"""
     from oracle.oracle import Reference
     if not Reference.available():
         pytest.skip("oracle/_ref not built (reference tree absent and no prebuilt copy)")
     return Reference()
+
+
+@pytest.fixture
+def ref(built, request):
+    """the reference's compiled transforms (oracle/_ref/libglava_ref.so) where they are built, their recorded results
+    elsewhere (tests/reference_record.py)"""
+    from oracle.oracle import Reference
+    from tests import reference_record
+    live = Reference.available()
+    return reference_record.ReferenceProxy(reference_record.Session(request, live), Reference() if live else None)
+
+
+@pytest.fixture
+def ref_record(built, request):
+    """results of the reference's shader tree (the test module's REF_SHADERS) run through oracle/glsl_interp.py: live
+    where the tree is present, recorded elsewhere (tests/reference_record.py)"""
+    from tests import reference_record
+    return reference_record.Session(request, os.path.isdir(request.module.REF_SHADERS))
 
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")

@@ -7,6 +7,7 @@ from the .frag / .glsl files themselves.  Since round 2 the pin is the reference
 import ctypes as C
 import json
 import os
+import zlib
 
 import numpy as np
 import pytest
@@ -14,9 +15,11 @@ import pytest
 import glava_b200 as g
 from oracle.oracle import params_from
 from tests.conftest import GOLDEN
+from tests.reference_record import same
 
 W, H, N = 96, 54, 512
 REF_SHADERS = "/root/reference/shaders/glava"
+OWN_CONFIG = os.path.join(os.path.dirname(g.__file__), "config")      # the reader's fallback on our side
 
 
 @pytest.fixture(scope="module")
@@ -137,8 +140,18 @@ def test_average_pass_frag(gold, F, win):
     assert _lsb(_unorm16(r / np.float32(F)), want) <= 1
 
 
-# ---- live: the interpreter against the oracle on a fresh configuration (build container only) ---------------------------------
-@pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
+# ---- the interpreter against the oracle on a fresh configuration (recorded where the reference tree is absent) ----------------
+def _interpret(module, w, h, tl, tr, **kw):
+    """one frame of the module's shaders from the reference tree, run by the interpreter"""
+    from oracle import glsl_interp as gi
+    prog = gi.ModuleProgram(REF_SHADERS, module, w, h, tl, tr, **kw)
+    got = np.zeros((h, w, 4), np.uint8)
+    for y in range(h):
+        for x in range(w):
+            got[y, x] = prog.pixel(x, y)
+    return got
+
+
 @pytest.mark.parametrize("module,gl_over,p_over", [
     ("bars", {"AMPLIFY": "30", "BAR_WIDTH": "3", "BAR_GAP": "1"}, dict(bars_amplify=30.0, bars_width=3.0, bars_gap=1.0)),
     ("radial", {"C_RADIUS": "9", "AMPLIFY": "20", "NBARS": "32"}, dict(radial_radius=9.0, radial_amplify=20.0, radial_nbars=32)),
@@ -146,22 +159,17 @@ def test_average_pass_frag(gold, F, win):
     ("graph", {"VSCALE": "30"}, dict(graph_vscale=30.0)),
     ("wave", {"AMPLIFY": "30"}, dict(wave_amplify=30.0)),
 ])
-def test_interpreter_live_against_the_oracle(orc, module, gl_over, p_over, built):
-    from oracle import glsl_interp as gi
+def test_interpreter_live_against_the_oracle(orc, ref_record, module, gl_over, p_over, built):
     w, h, n = 64, 40, 256
     p = orc.default_params(module, n=n, w=w, h=h, **p_over)
-    rng = np.random.default_rng(hash(module) % 1000)
+    rng = np.random.default_rng(zlib.crc32(module.encode()) % 1000)
     tl = orc.smooth_pass(p, (rng.random(n) ** 2 * 65535).astype(np.uint16))
     tr = orc.smooth_pass(p, (rng.random(n) ** 3 * 65535).astype(np.uint16))
     if module == "wave":
         tl = np.clip(tl.astype(int) // 4 + 24576, 0, 65535).astype(np.uint16)
     want = orc.raster(p, tl, tr)
-    prog = gi.ModuleProgram(REF_SHADERS, module, w, h, tl, tr, overrides=gl_over)
-    got = np.zeros_like(want)
-    for y in range(h):
-        for x in range(w):
-            got[y, x] = prog.pixel(x, y)
-    assert np.array_equal(got, want), (module, int((got != want).any(axis=2).sum()))
+    got = ref_record.call("interpret", lambda a, b: _interpret(module, w, h, a, b, overrides=gl_over), (tl, tr))
+    assert same(want, got), module
 
 
 @pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
@@ -172,7 +180,8 @@ def test_interpreter_reproduces_the_reference_known_answer(built):
     assert len(prog.stages) == 3 and prog.pixel(3, 2) == (0x55, 0, 0, 0x55)              # test_rc.glsl:27
 
 
-# ---- live: the config reader (glava_b200/csrc/config.cpp) against the shader semantics of the same config text ---------------
+# ---- the config reader (glava_b200/csrc/config.cpp) against the shader semantics of the same config text (recorded where the
+# reference tree is absent) ------------------------------------------------------------------------------------------------------
 USER_CONFIGS = {
     "bars": """
 #define BAR_WIDTH 3
@@ -255,20 +264,18 @@ USER_CONFIGS = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
 @pytest.mark.parametrize("module", sorted(USER_CONFIGS))
-def test_config_reader_agrees_with_the_shaders_on_a_user_config(orc, tmp_path, module, built):
+def test_config_reader_agrees_with_the_shaders_on_a_user_config(orc, ref_record, tmp_path, module, built):
     key, module = module, module.split(":")[0]
     """a user's <module>.glsl goes (a) through glava_b200_load_config -> parameters -> oracle raster and (b) as text through
     the reference's shaders in the interpreter: same pixels.  Covers colour literals / mix() gradients / constant
     vec4 colours / integer vs float macro values / parenthesised arithmetic in #defines."""
-    from oracle import glsl_interp as gi
     w, h, n = 72, 44, 256
     user = tmp_path / "user"
     user.mkdir()
     (user / "rc.glsl").write_text("#request mod %s\n#request setbufsize %d\n#request setgeometry 0 0 %d %d\n" % (module, n, w, h))
     (user / (module + ".glsl")).write_text(USER_CONFIGS[key])
-    p = g.load_config([str(user), REF_SHADERS])
+    p = g.load_config([str(user), OWN_CONFIG])
     assert p.module_name == module and (p.w, p.h, p.n) == (w, h, n)
     op = params_from(p)
     rng = np.random.default_rng(len(module))
@@ -277,28 +284,15 @@ def test_config_reader_agrees_with_the_shaders_on_a_user_config(orc, tmp_path, m
     if module == "wave":
         tl = np.clip(tl.astype(int) // 4 + 24576, 0, 65535).astype(np.uint16)
     want = orc.raster(op, tl, tr)
-    prog = gi.ModuleProgram(REF_SHADERS, module, w, h, tl, tr, config_dir=str(user))
-    got = np.zeros_like(want)
-    for y in range(h):
-        for x in range(w):
-            got[y, x] = prog.pixel(x, y)
-    assert want.any() and np.array_equal(got, want), (module, int((got != want).any(axis=2).sum()))
+    got = ref_record.call("interpret", lambda d, a, b: _interpret(module, w, h, a, b, config_dir=d), (str(user), tl, tr))
+    assert want.any() and same(want, got), module
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
-@pytest.mark.parametrize("F,win", [(5, 1), (3, 1), (2, 1), (1, 1), (4, 0)])
-def test_pipeline_b_chain_through_the_reference_pass_shaders(orc, F, win, built):
-    """the accelerated chain of one channel over several updates — R16 upload, K1 GL_MAX into gr_store, K2
-    gravity_pass.frag in place, K3 pass.frag into the ring slot, K4 average_pass.frag over the ring newest-first,
-    K5 smooth_pass.frag (render.c:2188-2303) — with every shader pass EXECUTED from the reference's source by the
-    interpreter, against orc_chan_update's restatement of the same chain: identical textures after every update."""
+def _pass_shader_chain(n, F, win, diff, bs):
+    """K1..K5 over the updates `bs`, every pass executed from the reference's util/*.frag by the interpreter; -> the K5
+    texture after every update"""
     from oracle import glsl_interp as gi
-    from oracle.oracle import OracleChannel
-    n = 128
     util = os.path.join(REF_SHADERS, "util")
-    p = orc.default_params("bars", n=n, accel_fft=1, avg_frames=F, avg_window=win)
-    ch = OracleChannel(orc, p)
-    rng = np.random.default_rng(F * 10 + win)
     hdr = dict(avg_frames=F, avg_window=win)
     grav = gi.load_stage(os.path.join(util, "gravity_pass.frag"), REF_SHADERS, None, **hdr)
     copy = gi.load_stage(os.path.join(util, "pass.frag"), REF_SHADERS, None, **hdr)
@@ -311,14 +305,11 @@ def test_pipeline_b_chain_through_the_reference_pass_shaders(orc, F, win, built)
             out[x] = gi.unorm16(sh.run(dict(uniforms), x, 0)["fragment"].v[0])
         return out
 
-    diff = np.float32(p.gravity_step) * (np.float32(1.0) / np.float32(p.ur))          # render.c:2224
     gr_store = np.zeros(n, np.uint16)
     ring = [np.zeros(n, np.uint16) for _ in range(F)]
     out_idx = 0
-    for u in range(2 * F + 3):
-        b = (rng.random(n) ** 2 * (1.3 if u % 3 else 0.2)).astype(np.float32)        # "transform_fft output", some > 1
-        spec = np.empty(n, np.float32); tex_o = np.empty(n, np.uint16)
-        orc.L.orc_chan_update(ch.h, C.byref(p), b.ctypes.data, 2, spec.ctypes.data, tex_o.ctypes.data)   # 2: `b` is transform_fft's output
+    outs = []
+    for b in bs:
         upload = _unorm16(b)                                                          # glTexImage1D GL_R16, render.c:521-524
         gr_store = np.maximum(gr_store, run(copy, {"tex": gi.Sampler1D(upload)}))     # K1: pass.frag blended with GL_MAX
         gr_store = run(grav, {"tex": gi.Sampler1D(gr_store), "diff": diff})           # K2 in place
@@ -328,17 +319,45 @@ def test_pipeline_b_chain_through_the_reference_pass_shaders(orc, F, win, built)
             uni = {f"t{t}": gi.Sampler1D(ring[(out_idx - t) % F]) for t in range(F)}  # t0 = most recent (render.c:2250-2255)
             tex = run(avg, uni)                                                       # K4
             out_idx = (out_idx + 1) % F
-        got = run(k5, {"tex": gi.Sampler1D(tex), "sz": n, "w": n})                    # K5
+        outs.append(run(k5, {"tex": gi.Sampler1D(tex), "sz": n, "w": n}))             # K5
+    return np.stack(outs)
+
+
+@pytest.mark.parametrize("F,win", [(5, 1), (3, 1), (2, 1), (1, 1), (4, 0)])
+def test_pipeline_b_chain_through_the_reference_pass_shaders(orc, ref_record, F, win, built):
+    """the accelerated chain of one channel over several updates — R16 upload, K1 GL_MAX into gr_store, K2
+    gravity_pass.frag in place, K3 pass.frag into the ring slot, K4 average_pass.frag over the ring newest-first,
+    K5 smooth_pass.frag (render.c:2188-2303) — with every shader pass EXECUTED from the reference's source by the
+    interpreter, against orc_chan_update's restatement of the same chain: identical textures after every update."""
+    from oracle.oracle import OracleChannel
+    n = 128
+    p = orc.default_params("bars", n=n, accel_fft=1, avg_frames=F, avg_window=win)
+    ch = OracleChannel(orc, p)
+    rng = np.random.default_rng(F * 10 + win)
+    bs = np.stack([(rng.random(n) ** 2 * (1.3 if u % 3 else 0.2)).astype(np.float32)  # "transform_fft output", some > 1
+                   for u in range(2 * F + 3)])
+    diff = np.float32(p.gravity_step) * (np.float32(1.0) / np.float32(p.ur))          # render.c:2224
+    gots = ref_record.call("pass_shader_chain", lambda d, b: _pass_shader_chain(n, F, win, d, b), (diff, bs), whole=True)
+    assert gots.shape == (2 * F + 3, n)
+    for u, (b, got) in enumerate(zip(bs, gots)):
+        spec = np.empty(n, np.float32); tex_o = np.empty(n, np.uint16)
+        orc.L.orc_chan_update(ch.h, C.byref(p), b.ctypes.data, 2, spec.ctypes.data, tex_o.ctypes.data)   # 2: `b` is transform_fft's output
         assert np.abs(got.astype(int) - tex_o.astype(int)).max() <= 1, (F, win, u)
         assert (got != tex_o).mean() < 0.02
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
-def test_k5_random_smooth_parameters_through_smooth_pass_frag(orc, orc_pm, tmp_path, built):
+def _smooth_pass_frag(d, sf, tex):
+    """util/smooth_pass.frag of the reference tree with user config dir d, run by the interpreter"""
+    from oracle import glsl_interp as gi
+    n = tex.shape[0]
+    sh = gi.load_stage(os.path.join(REF_SHADERS, "util", "smooth_pass.frag"), REF_SHADERS, None, config_dir=d, smooth_factor=sf)
+    return np.array([gi.unorm16(sh.run({"tex": gi.Sampler1D(tex), "sz": n, "w": n}, x, 0)["fragment"].v[0]) for x in range(n)], np.uint16)
+
+
+def test_k5_random_smooth_parameters_through_smooth_pass_frag(orc, orc_pm, ref_record, tmp_path, built):
     """smooth_pass.frag (K5) run from the reference's text with a random user smooth_parameters.glsl and setsmoothfactor,
     against the oracle and the product arithmetic (direct evaluation and the precomputed tap table): R16 texels within
     2 / 3 LSB16 (3e-5 / 5e-5 of full scale; the serial tap sums round differently by an ulp here and there)"""
-    from oracle import glsl_interp as gi
     from tests import emul
     rng = np.random.default_rng(31)
     n = 256
@@ -354,12 +373,11 @@ def test_k5_random_smooth_parameters_through_smooth_pass_frag(orc, orc_pm, tmp_p
         (user / "smooth_parameters.glsl").write_text(      # (a setsmoothfactor in rc.glsl would lose to smooth_parameters.glsl:72)
             f"#request setsmoothfactor {sf!r}\n#define SAMPLE_MODE {mode}\n#define ROUND_FORMULA {formula}\n#define SAMPLE_SCALE {scale!r}\n"
             f"#define SAMPLE_RANGE {rng_!r}\n#define SAMPLE_HYBRID_WEIGHT {hyb!r}\n")
-        p = g.load_config([str(user), REF_SHADERS])
+        p = g.load_config([str(user), OWN_CONFIG])
         p.n = n
         assert (p.sample_mode, p.round_formula) == (MODES[mode], FORMULAS[formula]) and p.smooth_factor == np.float32("%.6f" % sf)      # `#define _SMOOTH_FACTOR %.6f`
         tex = (rng.random(n) ** 2 * 65535).astype(np.uint16)
-        sh = gi.load_stage(os.path.join(REF_SHADERS, "util", "smooth_pass.frag"), REF_SHADERS, None, config_dir=str(user), smooth_factor=sf)
-        want = np.array([gi.unorm16(sh.run({"tex": gi.Sampler1D(tex), "sz": n, "w": n}, x, 0)["fragment"].v[0]) for x in range(n)], np.uint16)
+        want = ref_record.call("smooth_pass_frag", _smooth_pass_frag, (str(user), sf, tex), whole=True)
         assert want.any()
         assert _lsb(orc.smooth_pass(params_from(p), tex), want) <= 2, (trial, mode, formula)
         assert _lsb(emul.smooth(p, tex), want) <= 3 and _lsb(emul.k5_table(p, tex), want) <= 3, (trial, mode, formula)

@@ -1,5 +1,6 @@
 """A fixed slice of tools/fuzz_module_configs.py in the CPU tier: random user module configs as TEXT through the reference's
-own shaders (interpreter), through config reader + oracle, and through config reader + product arithmetic."""
+own shaders (interpreter; recorded where the reference tree is absent), through config reader + oracle, and through config
+reader + product arithmetic.  The reader falls back to the package's own config directory, not the reference's."""
 import importlib.util
 import os
 
@@ -8,8 +9,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SHADERS = "/root/reference/shaders/glava"
-
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
+OWN_CONFIG = os.path.join(ROOT, "glava_b200", "config")
 
 
 @pytest.fixture(scope="module")
@@ -25,10 +25,13 @@ def fuzz(built):
 # tools/fuzz_module_configs.py); 166 / 586 / 803 / 985:
 # the same with a smooth factor whose "%.6f" header literal differs from the request's float; the rest: a spread
 @pytest.mark.parametrize("seed", [207, 267, 131, 5, 12, 26, 33, 166, 586, 803, 985] + list(range(40, 66)))
-def test_random_module_config(fuzz, seed):
+def test_random_module_config(fuzz, ref_record, seed):
     module = ["bars", "radial", "circle", "graph", "wave"][seed % 5]
     w, h = [(40, 28), (41, 27), (38, 30)][seed % 3]
-    text, want, oracle, product = fuzz.run(seed, module, w, h, native=(seed % 4 != 3),
+
+    def frame(d, *args):
+        return ref_record.call("shader_frame", lambda *a: fuzz.shader_frame(d, *a[1:]), (d,) + args, whole=True)
+    text, want, oracle, product = fuzz.run(seed, module, w, h, native=(seed % 4 != 3), config_tail=OWN_CONFIG, frame=frame,
                                            smooth_in_shader=((1 + seed // 7 % 3) if (seed % 7 == 5 and module in ("bars", "radial", "circle", "graph")) else False))
     assert want.any(), text
     assert np.array_equal(oracle, want), (seed, module, text)

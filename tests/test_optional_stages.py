@@ -9,6 +9,7 @@ import pytest
 import glava_b200 as g
 from oracle.oracle import OracleStream, ext_from, params_from
 from tests.conftest import GOLDEN
+from tests.reference_record import same
 
 
 def test_transform_smooth_golden(orc):
@@ -25,10 +26,10 @@ def test_transform_smooth_live_reference_bit_exact(orc, ref, n):
     rng = np.random.default_rng(n)
     for d, ratio in ((0.01, 4.0), (0.05, 3.0), (0.3, 1.0)):
         x = (rng.random(n) ** 2).astype(np.float32); x[rng.random(n) < 0.3] = 0
-        assert np.array_equal(orc.transform_smooth(x, d, ratio), ref.smooth(x, d, ratio), equal_nan=True)
+        assert same(orc.transform_smooth(x, d, ratio), ref.smooth(x, d, ratio), equal_nan=True)
     silent = np.zeros(n, np.float32)                                         # every window empty: NaN over the head
     a, b = orc.transform_smooth(silent), ref.smooth(silent)
-    assert np.array_equal(a, b, equal_nan=True) and np.isnan(a[: n // 4]).all() and not np.isnan(a[n // 4:]).any()
+    assert same(a, b, equal_nan=True) and np.isnan(a[: n // 4]).all() and not np.isnan(a[n // 4:]).any()
 
 
 def test_bufscale_is_a_sequential_float_mean(orc):

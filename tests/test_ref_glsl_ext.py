@@ -21,7 +21,8 @@ def _auto_undef_removed(text):
 
 
 @pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
-def test_interpreter_front_end_is_token_identical_to_glsl_ext_c(ref, built):
+def test_interpreter_front_end_is_token_identical_to_glsl_ext_c(ref_live, built):
+    ref = ref_live
     import glob
     from oracle import glsl_interp as gi
     files = sorted(glob.glob(REF_SHADERS + "/*/*.frag"))
@@ -35,7 +36,8 @@ def test_interpreter_front_end_is_token_identical_to_glsl_ext_c(ref, built):
 
 
 @pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
-def test_shipped_rc_requests_as_the_reference_parses_them(ref, built):
+def test_shipped_rc_requests_as_the_reference_parses_them(ref_live, built):
+    ref = ref_live
     _, reqs = ref.ext_process(REF_SHADERS + "/rc.glsl", REF_SHADERS, None, REF_SHADERS)
     got = {r[0]: r[1:] for r in reqs}
     p = g.load_config([REF_SHADERS])

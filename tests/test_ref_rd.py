@@ -7,7 +7,11 @@ window backend (oracle/ref_shim.c, oracle/_ref/libglava_ref_rd.so):
   scaling, keyframe interpolation as the reference orchestrates them — against the oracle's restatement (orc_stream_*),
   which is what the kernels are tested against.
 
-Needs the reference tree (the shipped shaders are what rd_new loads) and an executable stack (skipped otherwise)."""
+rd_new / rd_update need the reference tree (the shipped shaders are what rd_new loads) and an executable stack; where
+either is missing their recorded results stand in (tests/reference_record.py: the configuration rd_new read, and every
+upload as digests of its floats and of its R16 texture — the comparisons here are bit for bit).  Our side reads the
+test's own files and the package's config directory, never the reference tree.  Tests that hand the reference's own
+shader text to either side still need the tree."""
 import os
 
 import numpy as np
@@ -15,28 +19,88 @@ import pytest
 
 import glava_b200 as g
 from oracle.oracle import OracleStream, OrcExt, ReferenceRenderer, params_from
+from tests.reference_record import Recorded, Session, same
 
 REF_SHADERS = "/root/reference/shaders/glava"
-pytestmark = [pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present"), pytest.mark.timeout(300)]
+OWN_CONFIG = os.path.join(os.path.dirname(g.__file__), "config")
+pytestmark = pytest.mark.timeout(300)
+needs_tree = pytest.mark.skipif(not os.path.isdir(REF_SHADERS), reason="reference tree not present")
+
+
+def _live():
+    return os.path.isdir(REF_SHADERS) and ReferenceRenderer.lib() is not None
+
+
+class _Renderer:
+    """ReferenceRenderer through a Session: .cfg as rd_new read it, frame() -> {texture: Recorded upload}"""
+
+    def __init__(self, s, paths, requests):
+        self.s = s
+        self.r = ReferenceRenderer(paths, requests=requests) if s.live else None
+        key = ["<reference tree>" if p == REF_SHADERS else p for p in paths]
+        self.cfg = s.call("rd_new", lambda *a: self.r.cfg, (key, list(requests)))
+        self.lb = np.zeros(self.cfg["bufsize"], np.float32)
+        self.rb = np.zeros(self.cfg["bufsize"], np.float32)
+
+    def set_rates(self, ur, fr):
+        self.s.call("set_rates", lambda *a: self.r.set_rates(ur, fr), (float(ur), float(fr)))
+
+    def frame(self, pcm_l=None, pcm_r=None):
+        if pcm_l is not None:
+            self.lb[:] = pcm_l; self.rb[:] = pcm_r
+
+        def live(*a):
+            with np.errstate(over="ignore", invalid="ignore"):         # (uploads of never-initialised keyframe buffers)
+                return {str(k): {"raw": Recorded.digest(v), "nan": Recorded.digest(v, True), "tex": Recorded.digest(_unorm16(v)),
+                                 "len": int(v.shape[0])} for k, v in self.r.frame(pcm_l, pcm_r).items()}
+        # (until two keyframes are pushed, interpolation uploads buffers the reference never initialised: check_live=False)
+        return {int(k): Recorded(d) for k, d in self.s.call("frame", live, (pcm_l, pcm_r), check_live=False).items()}
+
+    def close(self):
+        if self.r is not None:
+            self.r.close()
+
+
+@pytest.fixture
+def rd(built, request):
+    s = Session(request, _live())
+    return lambda paths, requests=(): _Renderer(s, paths, requests)
 
 
 @pytest.fixture(scope="module")
-def rd(built):
+def rd_live(built):
+    if not os.path.isdir(REF_SHADERS):
+        pytest.skip("reference tree not present")
     if ReferenceRenderer.lib() is None:
         pytest.skip("oracle/_ref/libglava_ref_rd.so not built or not loadable (needs an executable stack)")
     return ReferenceRenderer
 
 
+def _tex(up):
+    """the R16 texture of a recorded upload (GL's float -> R16 conversion of its floats)"""
+    return Recorded({"raw": up.d["tex"], "nan": up.d["tex"]})
+
+
 def _user_dir(path, files):
     """a user configuration directory the way `glava --copy-config` lays it out: the user's own files, symlinks to the
-    installed shaders / modules for everything else (render.c:1318-1320)"""
+    installed shaders / modules for everything else (render.c:1318-1320; only where the reference tree is present — only
+    the reference reads them)"""
     path.mkdir()
     for name, text in files.items():
         (path / name).write_text(text)
-    for entry in os.listdir(REF_SHADERS):
-        if entry not in files:
-            os.symlink(os.path.join(REF_SHADERS, entry), path / entry)
+    if os.path.isdir(REF_SHADERS):
+        for entry in os.listdir(REF_SHADERS):
+            if entry not in files:
+                os.symlink(os.path.join(REF_SHADERS, entry), path / entry)
     return str(path)
+
+
+def _own(path, files):
+    """the same user files for our config reader, which falls back to the package's config directory"""
+    path.mkdir()
+    for name, text in files.items():
+        (path / name).write_text(text)
+    return [str(path), OWN_CONFIG]
 
 
 def _unorm16(v):
@@ -65,16 +129,17 @@ CONFIGS = [
 
 @pytest.mark.parametrize("name,rc,sp,requests", CONFIGS, ids=[c[0] for c in CONFIGS])
 def test_config_reader_reads_what_rd_new_reads(rd, tmp_path, name, rc, sp, requests):
-    paths = [REF_SHADERS]
+    paths, ours = [REF_SHADERS], [OWN_CONFIG]
     if rc or sp:
         files = {"rc.glsl": rc or "#request mod bars\n"}
         if sp:
             files["smooth_parameters.glsl"] = sp
         paths = [_user_dir(tmp_path / "user", files), REF_SHADERS]
+        ours = _own(tmp_path / "own", files)
     r = rd(paths, requests=requests)
     try:
         c = r.cfg
-        p = g.load_config(paths, requests=requests)
+        p = g.load_config(ours, requests=requests)
         assert (p.n, p.rate_request, p.samplesize_request) == (c["bufsize"], c["rate"], c["samplesize"])
         assert p.channels == (1 if c["mirror_input"] else 2)
         assert (p.avg_frames, p.avg_window, p.smooth_pass, p.accel_fft) == (c["avg_frames"], c["avg_window"], c["smooth_pass"], c["accel_fft"])
@@ -93,11 +158,12 @@ def test_config_reader_reads_what_rd_new_reads(rd, tmp_path, name, rc, sp, reque
 
 def _chain_case(rd, tmp_path, extra_rc, ur, fr, pattern, seed):
     """pipeline A with the R16 texture taken straight from the upload (setsmoothpass false): reference uploads vs oracle"""
-    paths = [_user_dir(tmp_path / "u", {"rc.glsl": "#request mod bars\n#request setbufsize 1024\n#request setaccelfft false\n" + extra_rc,
-                                        "smooth_parameters.glsl": "#request setsmoothpass false\n"}), REF_SHADERS]
+    files = {"rc.glsl": "#request mod bars\n#request setbufsize 1024\n#request setaccelfft false\n" + extra_rc,
+             "smooth_parameters.glsl": "#request setsmoothpass false\n"}
+    paths = [_user_dir(tmp_path / "u", files), REF_SHADERS]
     r = rd(paths)
     try:
-        p = g.load_config(paths)
+        p = g.load_config(_own(tmp_path / "own", files))
         assert p.smooth_pass == 0 and p.accel_fft == 0
         p.ur = ur
         ext = OrcExt(bufscale=p.bufscale, interpolate=p.interpolate, fr=fr, transform_smooth=0, smooth_distance=0.01, smooth_ratio=4.0)
@@ -119,7 +185,7 @@ def _chain_case(rd, tmp_path, extra_rc, ur, fr, pattern, seed):
                 up = r.frame()
                 sl, sr, tl, tr = st.update(np.zeros(n, np.float32), np.zeros(n, np.float32), False)
             assert set(up) >= {0, 1}, (k, up.keys())
-            assert up[0].shape[0] == st.n
+            assert up[0].d["len"] == st.n
             interp_active = bool(p.interpolate) and ur / fr <= 0.9
             settled = pushed >= 2
             pushed += 1 if modified else 0
@@ -130,12 +196,12 @@ def _chain_case(rd, tmp_path, extra_rc, ur, fr, pattern, seed):
                 # stack copy (nlb / nrb, render.c:1765-1790) that is gone by the next frame, so a frame without new audio
                 # uploads the RAW box-averaged PCM — one untransformed frame flashes.  Oracle and product re-show the last
                 # spectrum, as the reference itself does when bufscale is 1 (lb / rb keep the transformed data).
-                assert np.array_equal(up[0], orc.bufscale(r.lb, p.bufscale)) and not np.array_equal(_unorm16(up[0]), tl)
+                assert same(orc.bufscale(r.lb, p.bufscale), up[0]) and not same(tl, _tex(up[0]))
                 checked += 1
                 continue
-            assert np.array_equal(_unorm16(up[0]), tl) and np.array_equal(_unorm16(up[1]), tr), (k, modified)
+            assert same(tl, _tex(up[0])) and same(tr, _tex(up[1])), (k, modified)
             if modified and not (p.interpolate and ur / fr <= 0.9):
-                assert np.array_equal(up[0], sl) and np.array_equal(up[1], sr), k      # the float chain result itself, bit for bit
+                assert same(sl, up[0]) and same(sr, up[1]), k                        # the float chain result itself, bit for bit
             checked += 1
         return checked
     finally:
@@ -167,10 +233,11 @@ def test_pipeline_b_uploads_transform_fft_only(rd, tmp_path):
     to the GL passes (render.c:2131-2180) — the oracle's `spec` in pipeline B is that buffer, bit for bit; interpolation is
     forced off for such a bind (render.c:2161-2168) even though rd_new's initialiser has it on"""
     from oracle.oracle import Oracle
-    paths = [_user_dir(tmp_path / "u", {"rc.glsl": "#request mod bars\n#request setbufsize 2048\n"}), REF_SHADERS]
+    files = {"rc.glsl": "#request mod bars\n#request setbufsize 2048\n"}
+    paths = [_user_dir(tmp_path / "u", files), REF_SHADERS]
     r = rd(paths)
     try:
-        p = g.load_config(paths)
+        p = g.load_config(_own(tmp_path / "own", files))
         assert p.accel_fft == 1 and p.interpolate == 1 and r.cfg["interpolate"] == 1
         p.ur = 30.0
         st = OracleStream(Oracle("libm"), params_from(p), OrcExt(bufscale=1, interpolate=1, fr=120.0, transform_smooth=0, smooth_distance=0.01, smooth_ratio=4.0))
@@ -180,7 +247,7 @@ def test_pipeline_b_uploads_transform_fft_only(rd, tmp_path):
             pl = (rng.standard_normal(p.n) * 0.2).astype(np.float32); pr = (rng.standard_normal(p.n) * 0.2).astype(np.float32)
             up = r.frame(pl, pr)
             sl, sr, _, _ = st.update(pl, pr, True)
-            assert np.array_equal(up[0], sl) and np.array_equal(up[1], sr), k
+            assert same(sl, up[0]) and same(sr, up[1]), k
     finally:
         r.close()
 
@@ -192,11 +259,12 @@ def test_wave_chain_window_wrange(rd, tmp_path):
     for extra, ur, fr, pattern in (("#request setinterpolate false\n", 86.0, 86.0, [1, 1, 0, 1]),
                                    ("", 30.0, 120.0, [1, 0, 1, 0, 0, 1, 0, 0, 0, 1, 0])):       # rd_new's initialiser: interpolation on
         d = tmp_path / ("w%d" % len(pattern))
-        paths = [_user_dir(d, {"rc.glsl": "#request mod wave\n#request setbufsize 1024\n" + extra}), REF_SHADERS]
+        files = {"rc.glsl": "#request mod wave\n#request setbufsize 1024\n" + extra}
+        paths = [_user_dir(d, files), REF_SHADERS]
         cli = ["setsmoothpass false"]             # (smooth_parameters.glsl cannot switch it off for wave; one CLI request can)
         r = rd(paths, requests=cli)
         try:
-            p = g.load_config(paths, requests=cli)
+            p = g.load_config(_own(tmp_path / ("own%d" % len(pattern)), files), requests=cli)
             assert p.smooth_pass == 0 and r.cfg["smooth_pass"] == 0
             p.ur = ur
             st = OracleStream(Oracle("libm"), params_from(p), OrcExt(bufscale=1, interpolate=p.interpolate, fr=fr, transform_smooth=0,
@@ -218,10 +286,10 @@ def test_wave_chain_window_wrange(rd, tmp_path):
                 pushed += 1 if modified else 0
                 if active and not settled:
                     continue
-                assert np.array_equal(_unorm16(up[0]), tl), (extra, k, modified)     # lerped or not: what the texture holds
+                assert same(tl, _tex(up[0])), (extra, k, modified)                   # lerped or not: what the texture holds
                 if modified and not active:
-                    assert np.array_equal(up[0], sl), (extra, k)
-                    assert np.array_equal(up[0], (pl + np.float32(1.0)) / np.float32(2.0))
+                    assert same(sl, up[0]), (extra, k)
+                    assert same((pl + np.float32(1.0)) / np.float32(2.0), up[0])
         finally:
             r.close()
 
@@ -258,7 +326,7 @@ def test_random_configs_against_rd_new(rd, tmp_path):
         r = rd(paths)
         try:
             c = r.cfg
-            p = g.load_config(paths)
+            p = g.load_config(_own(tmp_path / f"own{trial}", files))
             got = dict(bufsize=p.n, rate=p.rate_request, samplesize=p.samplesize_request, mirror_input=2 - p.channels,
                        avg_frames=p.avg_frames, avg_window=p.avg_window, smooth_pass=p.smooth_pass, accel_fft=p.accel_fft,
                        interpolate=p.interpolate, bufscale=p.bufscale, premultiply_alpha=p.premultiply_alpha, w=p.w, h=p.h)
@@ -273,7 +341,7 @@ def test_random_configs_against_rd_new(rd, tmp_path):
             r.close()
 
 
-def test_smooth_transform_after_fft_forces_the_cpu_order_chain(rd, tmp_path):
+def test_smooth_transform_after_fft_forces_the_cpu_order_chain(rd_live, tmp_path):
     """a module whose bind lists "smooth" after "fft" (render.c:1218-1286): under setaccelfft the reference can no longer
     leave gravity / average to the GL passes and runs fft -> gravity -> average -> smooth on the CPU (render.c:2143-2154);
     the uploaded buffer is the oracle's transform_smooth chain, NaN head included"""
@@ -289,7 +357,7 @@ def test_smooth_transform_after_fft_forces_the_cpu_order_chain(rd, tmp_path):
     os.unlink(d / "bars"); (d / "bars").mkdir()                           # a private copy of the module with the extra transform
     for f in os.listdir(os.path.join(REF_SHADERS, "bars")):
         (d / "bars" / f).write_text(src if f == "1.frag" else open(os.path.join(REF_SHADERS, "bars", f)).read())
-    r = rd(paths)
+    r = rd_live(paths)
     try:
         p = g.load_config(paths)
         assert p.accel_fft == 1 and p.smooth_distance == np.float32(0.02) and p.smooth_ratio == np.float32(3.0)
@@ -309,7 +377,7 @@ def test_smooth_transform_after_fft_forces_the_cpu_order_chain(rd, tmp_path):
 
 
 @pytest.mark.parametrize("accel", ["true", "false"])
-def test_smooth_transform_before_fft_runs_on_the_pcm(rd, tmp_path, accel):
+def test_smooth_transform_before_fft_runs_on_the_pcm(rd_live, tmp_path, accel):
     """a module whose bind lists "smooth" BEFORE "window" / "fft": handle_audio applies it on the CPU to the PCM ring, then
     meets "fft" and carries on as usual — GL passes under setaccelfft (the upload is transform_fft of the smoothed ring),
     the whole CPU chain otherwise (render.c:2131-2156).  transform_smooth = 2 in the oracle / product."""
@@ -325,7 +393,7 @@ def test_smooth_transform_before_fft_runs_on_the_pcm(rd, tmp_path, accel):
     os.unlink(d / "bars"); (d / "bars").mkdir()
     for f in os.listdir(os.path.join(REF_SHADERS, "bars")):
         (d / "bars" / f).write_text(src if f == "1.frag" else open(os.path.join(REF_SHADERS, "bars", f)).read())
-    r = rd(paths)
+    r = rd_live(paths)
     try:
         p = g.load_config(paths)
         assert p.accel_fft == (1 if accel == "true" else 0)
@@ -359,7 +427,7 @@ def test_smooth_transform_before_fft_runs_on_the_pcm(rd, tmp_path, accel):
     ("", "#request setsmoothpass false\n", (0, 1)),                                         # off where the shipped config sets it
     ("#request setsmoothpass false\n", "", (1, 2)),                                         # off in rc.glsl only: smoothed twice
 ])
-def test_stage1_header_is_built_before_its_includes_run_their_requests(rd, tmp_path, rc_extra, sp, state):
+def test_stage1_header_is_built_before_its_includes_run_their_requests(rd_live, tmp_path, rc_extra, sp, state):
     """shaderload forms `#define _PRE_SMOOTHED_AUDIO ...` (EBIND list, render.c:284-293) before ext_process runs the shader's
     own includes (:312): the module's FIRST shader believes smooth_pass as of the end of rc.glsl, the K5 pass follows the final
     value.  (params.smooth_pass, params.shader_pre_smoothed) must say exactly that."""
@@ -368,7 +436,7 @@ def test_stage1_header_is_built_before_its_includes_run_their_requests(rd, tmp_p
     if sp:
         files["smooth_parameters.glsl"] = open(os.path.join(REF_SHADERS, "smooth_parameters.glsl")).read() + sp
     paths = [_user_dir(tmp_path / "u", files), REF_SHADERS]
-    r = rd(paths)
+    r = rd_live(paths)
     try:
         p = g.load_config(paths)
         assert (p.smooth_pass, p.shader_pre_smoothed) == state
@@ -383,13 +451,13 @@ def test_stage1_header_is_built_before_its_includes_run_their_requests(rd, tmp_p
 
 
 @pytest.mark.parametrize("module", ["bars", "radial", "circle", "graph", "wave", "test"])
-def test_interpreter_consumes_what_rd_new_hands_to_the_glsl_compiler(rd, module):
+def test_interpreter_consumes_what_rd_new_hands_to_the_glsl_compiler(rd_live, module):
     """every fragment shader text the real rd_new passes to glShaderSource — injected header (render.c:315-327) + glsl_ext
     output — preprocesses to the same token stream as the interpreter's own pipeline (header_macros + ext_process) for the
     same file: module stages in order, then util/smooth_pass, gravity_pass, average_pass, pass.  Stages that `#error
     __disablestage` do so on both sides."""
     from oracle import glsl_interp as gi
-    r = rd([REF_SHADERS], requests=[f"mod {module}"])
+    r = rd_live([REF_SHADERS], requests=[f"mod {module}"])
     try:
         frags = r.sources[0::2]                                            # a raw vertex shader follows every fragment shader
         avg = r.cfg["avg_frames"]                                          # 5 from smooth_parameters.glsl; wave never reads it: 6
@@ -421,7 +489,7 @@ def test_interpreter_consumes_what_rd_new_hands_to_the_glsl_compiler(rd, module)
         r.close()
 
 
-def test_pipe_line_parser_against_the_one_inside_rd_update(rd, built):
+def test_pipe_line_parser_against_the_one_inside_rd_update(request, built):
     """the `--pipe` stdin parser is part of rd_update (render.c:1846-2005): the real one gets a pipe as stdin and one line per
     frame (oracle/ref_pipe_driver.py, a subprocess); the uniform writes it makes are what glava_b200_pipe_feed must store"""
     import json
@@ -433,10 +501,13 @@ def test_pipe_line_parser_against_the_one_inside_rd_update(rd, built):
              "fg =   ", "bg = #12x456", "amp = 1e3", "amp=-0.125", "f = 1,2", "b = #80", "bg = #123", "0.1,0.2,0.3,0.4", "amp = abc",
              "p = 7,8", "fg=#FFFFFFFF", "k=0x10", "on=1"]
     ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_pipe_driver.py"),
-                          json.dumps({"shaders": REF_SHADERS, "binds": binds, "lines": lines})], capture_output=True, text=True, timeout=120)
-    assert out.returncode == 0, out.stderr[-2000:]
-    ref = json.loads(next(ln for ln in out.stdout.splitlines() if ln.startswith("RESULT "))[7:])
+
+    def driver(binds, lines):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_pipe_driver.py"),
+                              json.dumps({"shaders": REF_SHADERS, "binds": binds, "lines": lines})], capture_output=True, text=True, timeout=120)
+        assert out.returncode == 0, out.stderr[-2000:]
+        return json.loads(next(ln for ln in out.stdout.splitlines() if ln.startswith("RESULT "))[7:])
+    ref = Session(request, _live()).call("pipe_driver", driver, (binds, lines))
     assert len(ref) == len(lines)
     with g.Pipe([f"{n}:{t}" for n, t in binds]) as pipe:
         width = {"vec4": 4, "vec3": 3, "vec2": 2, "float": 1}
@@ -462,22 +533,25 @@ def test_pipe_line_parser_against_the_one_inside_rd_update(rd, built):
     (["--pipe=x:mat4"], lambda: g.Pipe(["x:mat4"])), (["--pipe=fg", "--pipe=fg:float"], lambda: g.Pipe(["fg", "fg:float"])),
     (["--audio=nope"], lambda: __import__("glava_b200").audio.find_backend("nope")),
 ])
-def test_argument_errors_word_for_word(rd, args, ours):
+def test_argument_errors_word_for_word(request, built, args, ours):
     """what the reference's glava_entry prints when it rejects `--pipe NAME[:TYPE]` / `--audio NAME` is what the library
     reports for the same argument"""
     import subprocess
     import sys
     ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_entry_driver.py")] + args, capture_output=True, text=True, timeout=60)
-    theirs = out.stderr.strip()
-    assert theirs and out.returncode != 0
+
+    def driver(args):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_entry_driver.py")] + args, capture_output=True, text=True, timeout=60)
+        return [out.stderr.strip(), out.returncode]
+    theirs, rc = Session(request, _live()).call("entry_driver", driver, (args,))
+    assert theirs and rc != 0
     with pytest.raises(g.GlavaError) as e:
         ours()
     assert str(e.value).strip() == theirs
 
 
 @pytest.mark.parametrize("mirror", [False, True])
-def test_whole_program_fifo_to_uploads(rd, orc, tmp_path, mirror):
+def test_whole_program_fifo_to_uploads(rd_live, orc, tmp_path, mirror):
     """The whole reference program — glava_entry's argument parsing, rd_new, fifo.c's audio thread on a real named pipe, the
     frame loop's locked ring copy (glava.c:523-552), rd_update with the shipped setaccelfft — on the null driver for half a
     second (oracle/ref_program_driver.py).  Every frame that saw new audio uploads transform_fft of the rings as they stood;
@@ -539,7 +613,7 @@ def test_whole_program_fifo_to_uploads(rd, orc, tmp_path, mirror):
     assert max(seen["l"]) >= nchunks - 1                                   # the last chunk made it to the screen
 
 
-def test_whole_program_cpu_chain_state_by_state(rd, orc, tmp_path):
+def test_whole_program_cpu_chain_state_by_state(rd_live, orc, tmp_path):
     """the whole program with setaccelfft false: the writer paces its chunks, so the (much faster) frame loop sees EVERY ring
     state; each distinct upload must then be the oracle's fft -> gravity -> average chain advanced by exactly one ring update —
     the next chunk, or a zero slide where fifo.c's poll timed out in between (the log tells which).  `ur` stays at rd_new's

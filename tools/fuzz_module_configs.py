@@ -63,7 +63,14 @@ def gen(rng, module):
         D("MIN_THICKNESS", num(rng,1,2)); D("MAX_THICKNESS", num(rng,2,6)); D("BASE_COLOR", col(rng)); D("AMPLIFY", num(rng,10,60)); D("OUTLINE", col(rng))
     return "\n".join(L)+"\n"
 
-def run(seed, module, w, h, n=128, native=True, smooth_in_shader=False):
+def shader_frame(d, module, w, h, tl, tr, clear, hdr):
+    """the frame the reference's module shaders draw with user config dir d, run by the interpreter"""
+    prog=gi.ModuleProgram(REF, module, w, h, tl, tr, config_dir=d, clear_color=clear, **hdr)
+    return np.array([[prog.pixel(x,y) for x in range(w)] for y in range(h)],np.uint8)
+
+def run(seed, module, w, h, n=128, native=True, smooth_in_shader=False, config_tail=REF, frame=shader_frame):
+    """config_tail: the directory the reader falls back to after the user's; frame: shader_frame or a stand-in with its
+    arguments and result"""
     rng=np.random.default_rng(seed)
     text=gen(rng, module)
     d=tempfile.mkdtemp()
@@ -93,7 +100,7 @@ def run(seed, module, w, h, n=128, native=True, smooth_in_shader=False):
         hdr_extra = dict(pre_smoothed=1 if variant == 1 else 0, smooth_factor=sf)
         want_state = [(0, 0), (0, 1), (1, 2)][variant]
     open(d+"/rc.glsl","w").write(rc); open(f"{d}/{module}.glsl","w").write(text)
-    p=g.load_config([d, REF])
+    p=g.load_config([d, config_tail])
     n=p.n
     op=params_from(p)
     if smooth_in_shader and want_state != (1, 2):
@@ -103,8 +110,7 @@ def run(seed, module, w, h, n=128, native=True, smooth_in_shader=False):
     if module=="wave": tl=np.clip(tl.astype(int)//4+24576,0,65535).astype(np.uint16)
     hdr=dict(premultiply_alpha=p.premultiply_alpha, channels=p.channels, **hdr_extra)
     assert (p.smooth_pass, p.shader_pre_smoothed) == (want_state or (1, 0)), (p.smooth_pass, p.shader_pre_smoothed, want_state)
-    prog=gi.ModuleProgram(REF, module, w, h, tl, tr, config_dir=d, clear_color=clear, **hdr)
-    want=np.array([[prog.pixel(x,y) for x in range(w)] for y in range(h)],np.uint8)
+    want=frame(d, module, w, h, tl, tr, clear, hdr)
     o=orc.raster(op,tl,tr); e=emul.raster(p,tl,tr)
     return text, want, o, e
 
