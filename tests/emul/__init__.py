@@ -33,6 +33,7 @@ def lib():
         L.emul_lazy_k5.argtypes = [vp, i32, i32, vp, vp, vp]
         L.emul_lazy_epi_n.argtypes = [vp]
         L.emul_k5_table.argtypes = [vp, vp, vp]
+        L.emul_table_sizes.argtypes = [vp, i32, i32, vp]
         L.emul_bufscale.argtypes = [vp, i32, i32, vp]
         L.emul_transform_smooth.argtypes = [vp, i32, C.c_float, C.c_float]
         L.emul_upload.argtypes = [vp, vp, i32, C.c_float, C.c_float, i32, vp]
@@ -119,6 +120,16 @@ def lazy_k5(p, chan, path, av):
 
 def lazy_epi_n(p):
     return lib().emul_lazy_epi_n(C.byref(p))
+
+
+def table_sizes(p, target_rows=-105, texels_per_block=16):
+    """host table sizes the K5 launch structure is chosen from (capi.cu build_tables; the block shape defaults to its
+    own): dict(lazy_tab_bytes, lazy_blob_bytes, need_tile_rows, full_span, full_bytes); the lazy_* / need_* entries are
+    None for a module without a need-list"""
+    out = np.zeros(5, np.int64)
+    rc = lib().emul_table_sizes(C.byref(p), target_rows, texels_per_block, out.ctypes.data)
+    lazy = [int(v) for v in out[:3]] if rc == 0 else [None] * 3
+    return dict(lazy_tab_bytes=lazy[0], lazy_blob_bytes=lazy[1], need_tile_rows=lazy[2], full_span=int(out[3]), full_bytes=int(out[4]))
 
 
 def k5_table(p, tex):

@@ -327,6 +327,26 @@ int emul_lazy_epi_n(const glava_b200_params* pp) {
     build_lazy_tables(*pp, lists, &t);
     return t.epi_n;
 }
+// The host table sizes capi.cu's build_tables chooses a K5 launch structure from: out = {lazy tap-major table bytes, lazy
+// texel-major blob bytes of one channel, tallest need-block tile in rows (build_need_blocks with target_rows / tpb), full-
+// plane table's widest input span, full-plane table entry bytes}.  Returns -1 where the module has no need-list (the lazy
+// entries are then 0).
+int emul_table_sizes(const glava_b200_params* pp, int target_rows, int tpb, long long out[5]) {
+    const glava_b200_params& p = *pp;
+    for (int i = 0; i < 5; ++i) out[i] = 0;
+    K5TableHost k;
+    build_k5_table_host(p, &k);
+    out[3] = k.max_span; out[4] = (long long) (k.ent.size() * sizeof(K5Ent));
+    std::vector<int> lists[2];
+    if (!build_need_list(p, lists)) return -1;
+    LazyTables t;
+    build_lazy_tables(p, lists, &t);
+    NeedBlocks nb;
+    build_need_blocks(t, p.n, target_rows, tpb, &nb);
+    out[0] = (long long) (t.tab.size() * sizeof(TapEntry)); out[1] = (long long) t.blob; out[2] = nb.max_rows;
+    return 0;
+}
+
 // full-plane K5 of one plane through the per-block table, as k5_table_kernel does it (float staging, padded uniform loop)
 void emul_k5_table(const glava_b200_params* pp, const uint16_t* in, uint16_t* out) {
     const glava_b200_params& p = *pp;

@@ -243,3 +243,76 @@ def test_update_chain_random_parameters(orc_pm, built):
         peak = max(np.abs(s0).max(), 1e-30)
         assert np.abs(s0 - s1).max() / peak <= 1e-5, (trial, n)
         assert np.abs(t0.astype(int) - t1.astype(int)).max() <= 2, (trial, n)
+
+
+# ---- the need-list is complete: a lazy frame reads no texel outside it -----------------------------------------------
+_RASTER_OPTIONS = ([("bars", o) for o in (dict(bars_direction=1), dict(bars_invert=1), dict(bars_flip=1), dict(bars_mirror_yx=1),
+                                          dict(channels=1), dict(channels=1, bars_invert=1), dict(bars_outline_width=0.0),
+                                          dict(bars_width=3.0, bars_gap=2.0), dict(smooth_pass=0), dict(bars_width=1.0, bars_gap=0.0))]
+                   + [("radial", o) for o in (dict(radial_invert=1), dict(radial_off_x=40.0, radial_off_y=-25.0), dict(radial_nbars=37),
+                                              dict(radial_nbars=181), dict(radial_rotate=0.7), dict(radial_amplify=-120.0))]
+                   + [("graph", o) for o in (dict(graph_direction=-1), dict(graph_invert=1), dict(graph_draw_outline=1),
+                                             dict(graph_draw_highlight=0), dict(graph_join_channels=1))]
+                   + [(m, {}) for m in ("bars", "radial", "graph", "wave")])
+
+
+@pytest.mark.parametrize("w,h", [(320, 200), (333, 97), (802, 601)])
+@pytest.mark.parametrize("module,over", _RASTER_OPTIONS, ids=[f"{m}-{'-'.join(f'{k}={v}' for k, v in o.items()) or 'default'}" for m, o in _RASTER_OPTIONS])
+def test_lazy_frame_reads_only_need_list_texels(orc_pm, module, over, w, h, built):
+    """lazy_smooth = 1 smooths only the texels of emul.lazy_k5's list (tables.h build_need_list): every other texel of the
+    texture is stale on the device, so randomising all of them must leave the oracle's frame unchanged"""
+    n = 1024
+    p = g.default_params(module, n=n, w=w, h=h, lazy_smooth=1, **over)
+    op = params_from(p)
+    tl, tr = orc_pm.smooth_pass(op, _tex(n, 21)), orc_pm.smooth_pass(op, _tex(n, 22))
+    if module == "wave":
+        tl = (tl.astype(int) // 4 + 24576).astype(np.uint16)             # PCM-like values around 0.5
+    want = orc_pm.raster(op, tl, tr)
+    assert want.any()
+    rng = np.random.default_rng(w * h)
+    stale = []
+    for chan, t in ((0, tl), (1, tr)):
+        idx, _ = emul.lazy_k5(p, chan, 1, t)
+        keep = np.zeros(n, bool); keep[idx] = True
+        s = t.copy(); s[~keep] = rng.integers(0, 65536, int((~keep).sum()), dtype=np.uint16)
+        stale.append(s)
+    assert np.array_equal(orc_pm.raster(op, stale[0], stale[1]), want), (module, over, w, h)
+
+
+# ---- parameter sets that select a K5 fallback stay on their side of capi.cu's size thresholds -------------------------
+# capi.cu build_tables: lazy tap table <= 64 MB (:351), one channel's blob + the FFT buffers <= 112 KB for the one-kernel form
+# (:363), tallest need-block tile * 33 floats <= 200 KB for the shared-memory K5 tiles, else the L2 form (:382);
+# build_k5_table: full-plane table <= 256 MB and 2 spans <= 200 KB, else k5_planes_kernel evaluates the taps itself (:308).
+# tests/test_z_gpu_launch_structures.py runs these parameter sets on the device and counts their launches.
+MB = 1 << 20
+
+
+def _sizes(n, w=1920, **over):
+    return emul.table_sizes(g.default_params("bars", n=n, w=w, h=48, lazy_smooth=1, **over))
+
+
+@pytest.mark.parametrize("over", [dict(), dict(sample_mode=1)])
+def test_l2_fallback_parameters_exceed_the_tile_limit(over, built):
+    s = _sizes(16384, smooth_factor=0.1, **over)
+    assert s["lazy_tab_bytes"] <= 64 * MB and s["lazy_blob_bytes"] > 112 * 1024
+    assert s["need_tile_rows"] * 33 * 4 > 200 * 1024, s
+
+
+def test_full_plane_parameters_exceed_the_table_limit(built):
+    s = _sizes(16384, smooth_factor=0.3)
+    assert s["full_bytes"] > 256 * MB, s
+    assert s["need_tile_rows"] * 33 * 4 > 200 * 1024                   # (its lazy form: the L2 fallback)
+
+
+def test_split_below_4096_parameters_do_not_fit_next_to_the_fft(built):
+    s = _sizes(2048, w=7680)
+    assert s["lazy_blob_bytes"] > 112 * 1024 and s["need_tile_rows"] * 33 * 4 <= 200 * 1024, s
+
+
+@pytest.mark.parametrize("n", [512, 1024, 2048, 4096, 8192, 16384])
+def test_sweep_points_use_shared_memory_k5_tiles(n, built):
+    """every benchmarked shape at default parameters keeps its K5 out of the L2 fallback and its full-plane table uploaded"""
+    for w in (1280, 1920, 3840, 7680):
+        s = _sizes(n, w=w)
+        assert s["lazy_tab_bytes"] <= 64 * MB and s["need_tile_rows"] * 33 * 4 <= 200 * 1024, (n, w, s)
+        assert s["full_bytes"] <= 256 * MB and 2 * s["full_span"] * 4 <= 200 * 1024, (n, w, s)

@@ -165,7 +165,7 @@ def test_bad_arguments_fail_loudly(built):
         g.Renderer(g.default_params("bars", n=1000), batch=1)
 
 
-@pytest.mark.parametrize("n,w", [(1024, 320), (4096, 1920), (8192, 1920)])
+@pytest.mark.parametrize("n,w", [(1024, 320), (4096, 1920), (8192, 1920), (16384, 1920)])
 def test_kernel_variants_give_identical_textures_and_frames(built, monkeypatch, n, w):
     """the spectrum path exists in several launch structures (tuning knobs, DESIGN 6.2): plane-per-CTA kernel with in-kernel
     epilogue and K5; K5 as its own kernel over (texel, stream) pairs (through L2, or out of shared-memory tiles); the R16 state
@@ -178,7 +178,7 @@ def test_kernel_variants_give_identical_textures_and_frames(built, monkeypatch, 
 
     def run(env):
         for k in ("GLAVA_B200_K5_SPLIT", "GLAVA_B200_SPLIT_EPI", "GLAVA_B200_SPEC_OOP", "GLAVA_B200_SPEC_T", "GLAVA_B200_K5N_SMEM",
-                  "GLAVA_B200_K5N_ROWS", "GLAVA_B200_K5N_TPB", "GLAVA_B200_K5N_WARPS"):
+                  "GLAVA_B200_K5N_ROWS", "GLAVA_B200_K5N_TPB", "GLAVA_B200_K5N_WARPS", "GLAVA_B200_K5N_S", "GLAVA_B200_SPEC_CTAS_PER_SM"):
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():
             monkeypatch.setenv(k, v)
@@ -199,6 +199,7 @@ def test_kernel_variants_give_identical_textures_and_frames(built, monkeypatch, 
                 {"GLAVA_B200_K5_SPLIT": "0", "GLAVA_B200_SPEC_OOP": "1", "GLAVA_B200_SPEC_T": "128"},
                 # K5 over (texel, stream) pairs: through L2 from a transposed copy / out of shared-memory tiles over blocks of texels
                 {"GLAVA_B200_K5_SPLIT": "1", "GLAVA_B200_K5N_SMEM": "0"},
+                {"GLAVA_B200_K5_SPLIT": "1", "GLAVA_B200_K5N_SMEM": "0", "GLAVA_B200_K5N_S": "4"},     # (4 streams per lane: only through the knob)
                 {"GLAVA_B200_K5_SPLIT": "1", "GLAVA_B200_K5N_SMEM": "1"},
                 {"GLAVA_B200_K5_SPLIT": "1", "GLAVA_B200_K5N_SMEM": "1", "GLAVA_B200_K5N_ROWS": "64", "GLAVA_B200_K5N_TPB": "3", "GLAVA_B200_K5N_WARPS": "2"},
                 {}):                                                                                             # {} = this size's defaults
